@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — depth-frames/s (and Mvoxel-updates/s) of the semantic TSDF integrator hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload fast5|merged2|fast10] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload fast5|merged2|fast10] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic 640x480 depth+label frame (BASELINE.json
 configs[1] by default: 5 cm voxels, 21 classes, `fast` integrator).  Every step integrates a DIFFERENT
@@ -151,6 +151,9 @@ class _ReferenceSourceArm:
     def last_integrate_seconds(self):
         return self.integ.last_integrate_seconds()
 
+    def export(self):
+        return self.integ.export()
+
     def close(self):
         self.integ.close()
 
@@ -231,6 +234,34 @@ def peaks():
     return 6650.0, "fallback"
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, exp, seed=0):
+    """--dump-outputs: the map a caller of the timed path holds after its last step, as DIR/<name>.npy in float32 / float64, at most
+    DUMP_BYTES in all.  Blocks are sorted by block index, so that the files do not depend on allocation order; every block index is
+    written, the voxel fields for a fixed, seeded sample of the observed voxels (all of them when they fit)."""
+    os.makedirs(out_dir, exist_ok=True)
+    order = np.lexsort(exp["block_index"].T[::-1])
+    blocks = exp["block_index"][order].astype(np.float64)
+    b, v = np.nonzero(exp["tsdf_weight"][order] > 0)
+    C = exp["sem_priors"].shape[-1]
+    per_voxel = 8 * 2 + 4 * (3 + 4 + 4 + C)
+    n_max = (DUMP_BYTES - blocks.nbytes - 8) // per_voxel
+    observed = len(b)
+    if observed > n_max:
+        keep = np.sort(np.random.default_rng(seed).choice(observed, n_max, replace=False))
+        b, v = b[keep], v[keep]
+    rows = order[b]
+    arrays = {"block_index": blocks, "observed_voxels": np.array([observed], np.float64),
+              "voxel_index": np.stack([b, v], axis=1).astype(np.float64),     # (row of block_index, voxel within the block)
+              "tsdf_distance": exp["tsdf_distance"][rows, v], "tsdf_weight": exp["tsdf_weight"][rows, v],
+              "tsdf_rgba": exp["tsdf_rgba"][rows, v].astype(np.float32), "sem_label": exp["sem_label"][rows, v].astype(np.float32),
+              "sem_priors": exp["sem_priors"][rows, v], "sem_rgba": exp["sem_rgba"][rows, v].astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU implementation of the path - the faster of the oracle port and the reference-source
     build (oracle/_ref), at the thread count that is fastest on this host."""
@@ -252,6 +283,8 @@ def run_reference(args):
         if i >= args.warmup:
             t_total += integ.last_integrate_seconds()
             updates += st.voxel_updates
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, integ.export())
     integ.close()
     fps = args.steps / t_total
     line = {
@@ -368,6 +401,8 @@ def measure(args, workload, steps, warmup, ctx, with_cpu, profile_frames):
     launches, libcalls = prof["kernel_launches"], prof["library_calls"]
     clocks = sampler.stop() if rank == 0 else None
     blocks = integ.num_blocks()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, integ.export())
     if args.quick:
         integ.close()
         return {"workload": workload, "value": steps / (ms / 1e3), "ms_per_step": ms / steps, "quick": True,
@@ -671,6 +706,8 @@ def measure_frame_batches(args, workload, steps, warmup, ctx):
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, wall_ms = float(t[0]), float(t[1])
     blocks = base.num_blocks()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, base.export())
     base.close(); delta.close()
     if rank != 0:
         return None
@@ -715,6 +752,9 @@ def main():
     ap.add_argument("--quick", action="store_true", help="development aid: only the device-resident `value` leg, printed as a short line")
     ap.add_argument("--shim-e2e", type=int, default=1, help="N = 1: also time the C++ drop-in classes end to end (eager / lazy layer sync); 0 = skip")
     ap.add_argument("--extra-workloads", default="merged2", help="comma list of further workloads measured (briefly) into `workloads` at N = 1; '' = none")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the map they built (rank 0's) as DIR/<name>.npy: every block index and the voxel "
+                         "fields of a seeded sample of the observed voxels, at most 64 MB; the inputs are the same on every run")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -761,6 +801,7 @@ def main():
             # BASELINE.json configs[2] etc. in the same JSON line: a short run (frames are 10-100x heavier than the headline's)
             sub_args = argparse.Namespace(**vars(args))
             sub_args.sequences_per_gpu = 0
+            sub_args.dump_outputs = None
             extra[wl] = measure(sub_args, wl, min(args.steps, 30), 5, ctx, not args.no_cpu_baseline, min(args.profile_frames, 10))
     if world > 1 and args.sharding == "sequence" and args.extra_workloads:
         # N > 1: the headline above is N independent sequences (replicas, no collective on the data path).  The two modes that share ONE
@@ -773,10 +814,12 @@ def main():
                 return {"error": f"{type(e).__name__}: {e}"}
         sub = argparse.Namespace(**vars(args))
         sub.sequences_per_gpu = 0
+        sub.dump_outputs = None
         sub.sharding = "spatial"
         r1 = guarded(lambda: measure(sub, "merged2", 10, 3, ctx, False, 5))
         sub2 = argparse.Namespace(**vars(args))
         sub2.sharding = "frames"
+        sub2.dump_outputs = None
         r2 = guarded(lambda: measure_frame_batches(sub2, args.workload, 10, 3, ctx))
         extra["merged2_spatial"] = r1
         extra[f"{args.workload}_frame_batches"] = r2

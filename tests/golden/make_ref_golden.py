@@ -10,7 +10,13 @@ They travel to the GPU box (where neither /root/reference nor, necessarily, the 
   * the CUDA path          (tests/test_gpu_ref_golden.py, GPU)        - `fast` and `merged`: every digest, bit for bit (the product's
     default bundle order for `merged` is the reference's libstdc++ hash-map order).
 
-Regenerate (only in a container that has /root/reference):   make -C oracle ref && python tests/golden/make_ref_golden.py
+Given a reference checkout, `python tests/golden/make_ref_golden.py <checkout>` also records what the remaining comparisons with the
+reference's own code need, so that they run without it: digests of the random fuzz cases, of a 10 012-frame run and of an 8-thread run,
+the block counts of both layers, the outputs of the SemanticIntegratorBase helpers (ref_base_helpers.npz), the reference's label
+tables (label_csv/) with the reference reader's parse of each, and its ros_params.cpp on a few parameter files
+(ref_sources_golden.json).
+
+Regenerate where the reference exists:   make -C oracle ref && python tests/golden/make_ref_golden.py <checkout>
 """
 import hashlib
 import json
@@ -120,10 +126,138 @@ def run_case(name, make_integrator):
     return integ.export()
 
 
+GOLDEN_DIR = os.path.dirname(os.path.abspath(__file__))
+# the reference's label tables (kimera_semantics_ros/cfg), copied verbatim as data fixtures
+LABEL_CSV_DIR = os.path.join(GOLDEN_DIR, "label_csv")
+SOURCES_GOLDEN = os.path.join(GOLDEN_DIR, "ref_sources_golden.json")
+HELPERS_GOLDEN = os.path.join(GOLDEN_DIR, "ref_base_helpers.npz")
+CSV_PLACEHOLDER = "{csv}"      # stands for the label CSV path inside recorded ros_params output
+THREADS_CASE = "fast_fullsize_640x480_5cm_4f"
+
+
+def helper_inputs(n=200, seed=7):
+    """Random prior / frequency rows for the SemanticIntegratorBase helpers, p = 0.8 (case fast_p08)."""
+    rng = np.random.default_rng(seed)
+    priors = (-rng.uniform(0.1, 40.0, (n, C21))).astype(np.float32)
+    freqs = rng.integers(0, 6, (n, C21)).astype(np.float32)
+    freqs[::5] = np.eye(C21, dtype=np.float32)[rng.integers(0, C21, len(freqs[::5]))]      # one-hot rows, as `fast` produces them
+    return case_config("fast_p08"), priors, freqs
+
+
+def full_reset_frames(n_frames=10012, points_per_frame=24, seed=5):
+    """Many tiny clouds: drives the ApproxHashSet offset through its full-reset threshold (10 000 resets)."""
+    rng = np.random.default_rng(seed)
+    for f in range(n_frames):
+        T = synth.pose(f % 300)
+        xyz = np.stack([rng.uniform(-0.4, 0.4, points_per_frame), rng.uniform(-0.3, 0.3, points_per_frame),
+                        rng.uniform(0.8, 1.6, points_per_frame)], axis=1).astype(np.float32)
+        lab = rng.integers(0, 20, points_per_frame).astype(np.uint8)
+        yield T, xyz, lab
+
+
+def full_reset_config():
+    return make_config(FAST, 0.10, C21, max_points=64)
+
+
+def run_full_reset(integ, cfg):
+    pal = np.array([[cfg.label_color[l][k] for k in range(4)] for l in range(256)], np.uint8)
+    if hasattr(integ, "set_color_to_label"):
+        integ.set_color_to_label(*color_table(cfg))
+    for T, xyz, lab in full_reset_frames():
+        integ.integrate_points(T, xyz, rgba=np.ascontiguousarray(pal[lab]))
+    return integ.export()
+
+
+ROS_PARAM_TEXTS = [
+    "method: merged\nsemantic_color_mode: semantic_probability\nsemantic_measurement_probability: 0.75\ndynamic_semantic_labels: [20, 3, 7]\n",
+    "dynamic_semantic_labels: []\n",                                  # every default: fast, colour mode "color", p = 0.9
+    "semantic_color_mode: rainbow\ndynamic_semantic_labels: [1]\n",
+    "method: fast\n",                                                 # CHECK(getParam("dynamic_semantic_labels")) ros_params.cpp:69
+]
+SMALL_LABEL_CSV = "name,red,green,blue,alpha,id\nfloor,10,20,30,255,1\nwall,40,50,60,255,2\n"
+
+
+def _in_subprocess(expr, arg):
+    """The reference aborts on malformed input (CHECK / LOG(FATAL)), so each call runs in its own process."""
+    import subprocess
+    r = subprocess.run([sys.executable, "-c", f"import sys; from oracle import ref_py; sys.stdout.write({expr}(sys.argv[1]))", arg],
+                       capture_output=True, text=True, cwd=ROOT)
+    # the last log line without its "F <source path>:<line>] " prefix
+    last = r.stderr.strip().splitlines()[-1] if r.stderr.strip() else ""
+    return {"ok": r.returncode == 0, "stdout": r.stdout, "error": last.split("] ", 1)[-1]}
+
+
+def reference_records(ref_dir):
+    """Everything else the tests compare with the reference's own code, recorded from oracle/_ref and the reference checkout."""
+    import shutil
+    import tempfile
+    import fuzz_cases
+    from oracle.ref_py import RefHybridIntegrator
+    rec = {}
+    fuzz = {}
+    for seed in range(24):
+        cfg, frames_ = fuzz_cases.make_case(seed)
+        ref = RefHybridIntegrator(cfg)
+        with fuzz_cases.quiet_stderr():
+            for T, pts, rgba, freespace in frames_:
+                ref.integrate_points(T, pts, rgba=rgba, freespace=freespace)
+        fuzz[str(seed)] = digest(ref.export())
+    rec["fuzz"] = fuzz
+    cfg = case_config("fast_default_3f")
+    ref = RefHybridIntegrator(cfg)
+    for T, xyz, rgba, fs in case_frames("fast_default_3f", cfg):
+        ref.integrate_points(T, xyz, rgba=rgba, freespace=fs)
+    rec["block_counts_fast_default_3f"] = {"tsdf": ref.num_blocks(), "semantic": ref.num_semantic_blocks()}
+    cfg = full_reset_config()
+    rec["full_reset_10012_frames"] = digest(run_full_reset(RefHybridIntegrator(cfg), cfg))
+
+    def threads(n):
+        def make(cfg):
+            cfg.integrator_threads = n
+            return RefHybridIntegrator(cfg)
+        return make
+    rec["threads8_" + THREADS_CASE] = digest(run_case(THREADS_CASE, threads(8)))
+
+    os.makedirs(LABEL_CSV_DIR, exist_ok=True)
+    cfg_dir = os.path.join(ref_dir, "kimera_semantics_ros", "cfg")
+    csv = {}
+    for name in sorted(os.listdir(cfg_dir)):
+        if name.endswith("_mapping.csv") or name == "simulation.csv":
+            shutil.copyfile(os.path.join(cfg_dir, name), os.path.join(LABEL_CSV_DIR, name))
+            csv[name] = _in_subprocess("ref_py.csv_dump", os.path.join(LABEL_CSV_DIR, name))
+    rec["label_csv"] = csv
+    params = []
+    with tempfile.TemporaryDirectory() as td:
+        path = os.path.join(td, "labels.csv")
+        open(path, "w").write(SMALL_LABEL_CSV)
+        for text in ROS_PARAM_TEXTS:
+            r = _in_subprocess("ref_py.ros_params", text + f"semantic_label_2_color_csv_filepath: {path}\n")
+            r["stdout"] = r["stdout"].replace(path, CSV_PLACEHOLDER)
+            params.append(dict(r, text=text))
+    rec["ros_params"] = params
+    return rec
+
+
+def record_base_helpers():
+    from oracle.ref_py import RefHybridIntegrator
+    cfg, priors, freqs = helper_inputs()
+    ref = RefHybridIntegrator(cfg)
+    L, lm, ln = ref.log_likelihood()
+    upd = np.stack([ref.update_probabilities(freqs[k], priors[k]) for k in range(len(priors))])
+    np.savez_compressed(HELPERS_GOLDEN, log_likelihood=L, log_match=np.float32(lm), log_non_match=np.float32(ln), updated=upd,
+                        label_rgba=np.stack([ref.label_color(l) for l in range(C21)]),
+                        normalized=np.stack([ref.normalize_probabilities(u) for u in upd]))
+
+
 if __name__ == "__main__":
+    # usage: python tests/golden/make_ref_golden.py <reference checkout>   (after `make -C oracle ref REF=<checkout>/kimera_semantics ...`)
     from oracle.ref_py import RefHybridIntegrator, available
     assert available(), "build oracle/_ref first: make -C oracle ref"
     out = {name: digest(run_case(name, RefHybridIntegrator)) for name in CASES}
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_hybrid_golden.json")
+    path = os.path.join(GOLDEN_DIR, "ref_hybrid_golden.json")
     json.dump(out, open(path, "w"), indent=1, sort_keys=True)
     print("wrote", path, len(out), "cases")
+    if len(sys.argv) > 1:
+        json.dump(reference_records(sys.argv[1]), open(SOURCES_GOLDEN, "w"), indent=1, sort_keys=True)
+        record_base_helpers()
+        print("wrote", SOURCES_GOLDEN, HELPERS_GOLDEN, LABEL_CSV_DIR)

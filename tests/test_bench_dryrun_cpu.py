@@ -65,6 +65,9 @@ class FakeDeviceIntegrator:
     def sync(self):
         pass
 
+    def export(self):
+        return self.o.export()
+
     def close(self):
         self.o.close()
 
@@ -81,10 +84,7 @@ class FakeEvent:
         return max(1e-3, (other.t - self.t) * 1e3)
 
 
-@pytest.mark.parametrize("workload,extra", [("fast10", []), ("merged5", ["--merged-bundle-order", "libstdcxx", "--hot-voxels", "2"])])
-def test_bench_main_dry_run_produces_a_complete_line(monkeypatch, workload, extra):
-    if workload == "merged5":
-        monkeypatch.setitem(bench.WORKLOADS, "merged5", (capi.KSG_INTEGRATOR_MERGED, 160, 120, 0.10, 21, 16 << 20, 8192))   # small frames
+def fake_device(monkeypatch):
     monkeypatch.setattr(capi, "Integrator", FakeDeviceIntegrator)
     monkeypatch.setattr(torch.cuda, "is_available", lambda: True)
     monkeypatch.setattr(torch.cuda, "set_device", lambda d: None)
@@ -97,6 +97,13 @@ def test_bench_main_dry_run_produces_a_complete_line(monkeypatch, workload, extr
     monkeypatch.setattr(torch.Tensor, "pin_memory", lambda self, *a, **k: self)
     real_tensor = torch.tensor
     monkeypatch.setattr(torch, "tensor", lambda *a, **k: real_tensor(*a, **{kk: vv for kk, vv in k.items() if kk != "device"}))
+
+
+@pytest.mark.parametrize("workload,extra", [("fast10", []), ("merged5", ["--merged-bundle-order", "libstdcxx", "--hot-voxels", "2"])])
+def test_bench_main_dry_run_produces_a_complete_line(monkeypatch, workload, extra):
+    if workload == "merged5":
+        monkeypatch.setitem(bench.WORKLOADS, "merged5", (capi.KSG_INTEGRATOR_MERGED, 160, 120, 0.10, 21, 16 << 20, 8192))   # small frames
+    fake_device(monkeypatch)
     monkeypatch.setattr(sys, "argv", ["bench.py", "--workload", workload, "--steps", "4", "--warmup", "3", "--profile-frames", "2", "--sequences-per-gpu", "2", "--shim-e2e", "0",
                                       "--extra-workloads", "fast10" if workload != "fast10" else "merged5"] + extra)
     monkeypatch.setattr(bench, "best_cpu_arm", lambda wl, fr, cam: ("port", 1, {"port@1": 1.0}))
@@ -121,3 +128,37 @@ def test_bench_main_dry_run_produces_a_complete_line(monkeypatch, workload, extr
     assert line["config"]["merged_bundle_order"] == "libstdcxx"
     assert line["config"]["hot_voxel_mode"] == (2 if extra else 0)
     assert line["gpu_launches"] > 0
+
+
+@pytest.mark.parametrize("limit", [None, 1 << 20])
+def test_dump_outputs_is_the_map_after_exactly_the_timed_steps(monkeypatch, tmp_path, limit):
+    """--dump-outputs writes the map of the timed integrator: warm-up + --steps frames, the same on every run, float32 / float64 only,
+    within the byte budget (a seeded sample of the observed voxels when the map does not fit)."""
+    fake_device(monkeypatch)
+    if limit:
+        monkeypatch.setattr(bench, "DUMP_BYTES", limit)
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--workload", "fast10", "--steps", "5", "--warmup", "3", "--quick", "--dump-outputs", str(out)])
+        with redirect_stdout(io.StringIO()):
+            bench.main()
+        dumps.append({p.stem: np.load(p) for p in sorted(out.iterdir())})
+    a, b = dumps
+    assert sorted(a) == sorted(b) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= bench.DUMP_BYTES
+    cam, frames = bench.gen_frames("fast10", 3 + 5)
+    ora = OracleIntegrator(bench.make_cfg("fast10"))
+    for depth, label, T in frames:
+        ora.integrate_depth(T, depth, label, cam.K)
+    exp = ora.export()
+    order = np.lexsort(exp["block_index"].T[::-1])
+    assert np.array_equal(a["block_index"], exp["block_index"][order])
+    observed = exp["tsdf_weight"][order] > 0
+    assert a["observed_voxels"][0] == observed.sum()
+    assert (len(a["voxel_index"]) < observed.sum()) == bool(limit)
+    rows, vox = a["voxel_index"][:, 0].astype(int), a["voxel_index"][:, 1].astype(int)
+    assert observed[rows, vox].all()
+    for k in ("tsdf_distance", "tsdf_weight", "sem_priors", "sem_label"):
+        assert np.array_equal(a[k], exp[k][order][rows, vox]), k
