@@ -355,7 +355,7 @@ int64_t ksg_debug_tile_times(ksg_integrator* h, int32_t enable, int64_t capacity
  * segments allocated + new blocks constructed, out[56] records scattered (kernel end); out[64..79]: maxima / counts gathered inside the
  * kernel (longest single ray set-up / evaluation in clocks, rays evaluated, blocks evaluated / materialised, ...); *sweeps = sweeps of that
  * frame, *clock_khz = SM clock the stamps count in.  Returns the number of slots written (80) or 0. */
-int64_t ksg_debug_fast_timeline(ksg_integrator* h, int64_t* out80 /* 64 time marks + 16 debug maxima / counts */, int64_t* sweeps, double* clock_khz);
+int64_t ksg_debug_fast_timeline(ksg_integrator* h, int64_t* out112 /* 64 time marks + 16 debug maxima / counts + 32 solver counters */, int64_t* sweeps, double* clock_khz);
 
 /* Debug aid for the next optimisation (not on the integration path): evaluates  s <- fl(s + terms[k]), k = 0..n-1  (s0 < 0, terms <= 0,
  * float32, round to nearest even) with ONE warp as an exact associative scan (lanes = records, csrc/ksg_chain.cuh) and returns the

@@ -472,7 +472,7 @@ class Integrator:
 
     def fast_timeline(self) -> Dict[str, object]:
         """Phase boundaries of the last frame's persistent solve kernel in microseconds from its start (fast integrator, profiling on)."""
-        out = (C.c_int64 * 80)()
+        out = (C.c_int64 * 112)()
         sweeps, khz = C.c_int64(), C.c_double()
         n = int(self.lib.ksg_debug_fast_timeline(self.handle, out, C.byref(sweeps), C.byref(khz)))
         if n == 0:
@@ -491,7 +491,10 @@ class Integrator:
                           "ray_evals_that_changed": t[71], "max_shared_slot_visitors": t[72], "shared_slot_visitors": t[73],
                           "shared_slots": t[74], "rays": t[75],
                           "max_setup_after_loads_us": t[76] / (khz.value / 1e3), "max_setup_after_init_us": t[77] / (khz.value / 1e3),
-                          "max_setup_after_loop_us": t[78] / (khz.value / 1e3), "max_eval_first_block_loads_us": t[79] / (khz.value / 1e3)}}
+                          "max_setup_after_loop_us": t[78] / (khz.value / 1e3), "max_eval_first_block_loads_us": t[79] / (khz.value / 1e3),
+                          "overflow_entries": t[80], "max_slot_count": t[81], "max_overflow_chain_walked": t[82],
+                          "sweep_clean_rays": [t[84 + 2 * i] for i in range(max(0, min(ns, 14)))],
+                          "sweep_ray_evals": [t[85 + 2 * i] for i in range(max(0, min(ns, 14)))]}}
 
     def sync(self):
         self._check(self.lib.ksg_sync(self.handle), "ksg_sync")

@@ -150,6 +150,7 @@ struct ksg_integrator {
   bool fast_v2 = false;
   FastCounters* d_fc = nullptr;
   FastCounters* h_fc = nullptr;      // pinned
+  long long* d_prof = nullptr;       // [kProfSlots] solver counters of the last profiled frame (allocated when profiling is first enabled)
   int *blk_cnt = nullptr, *blk_off = nullptr, *warp_cnt = nullptr, *warp_off = nullptr, *seq_of_i = nullptr;
   uint32_t* keys32 = nullptr;
   int *tile_cnt = nullptr, *tile_slot = nullptr;
@@ -276,7 +277,7 @@ void free_all(ksg_integrator* h) {
                   h->ray_color, h->nsteps, h->H, h->L, h->ray_state, h->ext_off, h->eval_sweep, h->ob.slot_stamp, h->ob.cand_pos, h->ob.bkt, h->ob.cand_val, h->ob.cand_order,
                   h->ob.cand_next, h->ob.table, h->ks_sorted, h->seq_sorted, h->bstart, h->bundle_f, h->hist,
                   h->tmp, h->tmp4, h->b_key, h->b_base, h->bord_hash, h->bord_scratch, h->d_scan_tot, h->bundle_f2, h->d_hot_segs, h->d_hot_counts, h->d_hot_chunk_seg, h->d_hot_guess, h->d_hot_sums,
-                  h->d_hot_tables, h->d_hot_prior, h->d_hot_same, h->tile_debug, h->d_gridbar, h->d_fc, h->blk_cnt, h->blk_off, h->warp_cnt, h->warp_off, h->seq_of_i, h->keys32,
+                  h->d_hot_tables, h->d_hot_prior, h->d_hot_same, h->tile_debug, h->d_gridbar, h->d_fc, h->d_prof, h->blk_cnt, h->blk_off, h->warp_cnt, h->warp_off, h->seq_of_i, h->keys32,
                   h->tile_cnt, h->tile_slot, h->tile_list, h->cand16, h->ovf, h->rayrec, h->mixed_list, h->m_list, h->blk_run, h->stamp64, h->d_log_head, h->d_log_prior, h->vq.long_items, h->vq.counters, h->rec_a, h->rec_b, h->tile_begin, h->cub_temp, h->d_in, h->d_exp, h->d_exp_slots};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->h_cnt_base) cudaFreeHost(h->h_cnt_base);
@@ -520,6 +521,7 @@ int integrate_fast_v2(ksg_integrator* h, const InputDesc& in, const FrameIn& fin
   f.vec_ok = in.d_depth ? (((uintptr_t)in.d_depth % 16 == 0 && (uintptr_t)in.d_label_img % 4 == 0) ? 1 : 0) : 0;
   f.frame_stamp = h->frame_stamp;
   f.profile = h->profiling ? 1 : 0;
+  f.prof = h->d_prof;
   f.seq_of_i = sorted ? h->seq_of_i : nullptr;
   f.block_cnt = h->blk_cnt; f.block_off = h->blk_off; f.warp_cnt = h->warp_cnt; f.warp_off = h->warp_off;
   f.pt_pG = h->pt_pG; f.pt_label = h->pt_label; f.pt_flags = h->pt_flags; f.pt_color = h->pt_color; f.pt_key = h->pt_key;
@@ -540,6 +542,7 @@ int integrate_fast_v2(ksg_integrator* h, const InputDesc& in, const FrameIn& fin
   if (h->profiling) {
     cudaEventRecord(h->ev[0], s);
     KSG_CUDA(cudaMemsetAsync(h->d_fc->dbg, 0, sizeof(h->d_fc->dbg), s));
+    KSG_CUDA(cudaMemsetAsync(h->d_prof, 0, sizeof(long long) * kProfSlots, s));
   }
   KSG_CUDA(cudaMemsetAsync(h->clear_ff, 0xFF, (size_t)kSetSize * 16, s));
   KSG_CUDA(cudaMemsetAsync(h->clear_00, 0x00, (size_t)kSetSize * (s3 ? 13 : 5), s));
@@ -2189,6 +2192,10 @@ int32_t ksg_set_profiling(ksg_integrator* h, int32_t enable) {
   if (!h) return KSG_ERR_INVALID_ARGUMENT;
   cudaSetDevice(h->device);
   if (enable && !h->ev[0]) for (auto& e : h->ev) cudaEventCreate(&e);
+  if (enable && h->d_fc && !h->d_prof) {
+    if (cudaMalloc(&h->d_prof, sizeof(long long) * kProfSlots) != cudaSuccess) { h->d_prof = nullptr; return KSG_ERR_CUDA; }
+    cudaMemset(h->d_prof, 0, sizeof(long long) * kProfSlots);
+  }
   h->profiling = enable != 0;
   for (double& m : h->phase_ms) m = 0.0;
   h->prof_frames = 0; h->n_launches = 0; h->n_libcalls = 0;
@@ -2247,9 +2254,12 @@ int64_t ksg_debug_fast_timeline(ksg_integrator* h, int64_t* out64, int64_t* swee
   if (h->n_pend > 0) finish_frame(h, nullptr);
   for (int i = 0; i < kTimelineSlots; ++i) out64[i] = (int64_t)h->h_fc->timeline[i];
   for (int i = 0; i < 16; ++i) out64[kTimelineSlots + i] = (int64_t)h->h_fc->dbg[i];
+  long long prof[kProfSlots] = {};
+  if (h->d_prof) cudaMemcpy(prof, h->d_prof, sizeof(prof), cudaMemcpyDeviceToHost);
+  for (int i = 0; i < kProfSlots; ++i) out64[kTimelineSlots + 16 + i] = (int64_t)prof[i];
   if (sweeps) *sweeps = h->h_fc->sweeps_last;
   if (clock_khz) *clock_khz = h->clock_khz;
-  return kTimelineSlots + 16;
+  return kTimelineSlots + 16 + kProfSlots;
 }
 
 int32_t ksg_clear_map(ksg_integrator* h) {

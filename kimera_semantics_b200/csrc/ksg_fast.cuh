@@ -29,6 +29,11 @@ static constexpr int kSolveThreads = 1024;     // one CTA per SM: a grid barrier
 static constexpr int kFastKeyCap = 4096;      // update records of one tile sorted in shared memory (more: sorted in place in global memory)
 static constexpr int kFastPref = 1024;        // ... and whose per-record operands (point, label, colour) are prefetched into shared memory
 static constexpr int kTimelineSlots = 64;
+// profiling-only solver counters (FastFrame::prof, not part of FastCounters, which is copied back every frame):
+//   [0] overflow entries of the frame, [1] largest slot count, [2] longest overflow chain walked by an evaluation,
+//   [4 + 2 i] rays of sweep i found clean by the dirty check alone, [5 + 2 i] rays of sweep i evaluated (i < kProfSweeps)
+static constexpr int kProfSlots = 32;
+static constexpr int kProfSweeps = (kProfSlots - 4) / 2;
 
 struct FastCounters {      // device-resident state of the frame driver (persistent across frames)
   unsigned int ticket_count, ticket_eval;   // "last block done" tickets
@@ -91,6 +96,7 @@ struct FastFrame {
   int vec_ok;                // depth / label pointers allow 128-bit / 32-bit vector loads
   int frame_stamp;
   int profile;
+  long long* prof;           // [kProfSlots] (profiling only)
   const int* seq_of_i;       // "sorted" order mode: sequence position of input index i, else NULL (mixed: closed form)
   int* block_cnt; int* block_off;     // finite pixels per 1024-pixel block
   int* warp_cnt; int* warp_off;       // cast points per 32 sequence positions
@@ -430,17 +436,20 @@ __device__ __forceinline__ void warp_sort_i32(int* a, int n, int lane) {
   int n2 = 1;
   while (n2 < n) n2 <<= 1;
   const int half = n2 >> 1;
-  for (int k = 2; k <= n2; k <<= 1) {
-    const int hk = k >> 1;
+  // k and j are powers of two: shifts and masks instead of integer divisions (the sort of a slot with a few hundred visitors is
+  // ~360 dependent compare-exchange rounds of one warp, and the divisions were most of each round)
+  for (int lk = 1; (1 << lk) <= n2; ++lk) {
+    const int k = 1 << lk, lhk = lk - 1;
     for (int t = lane; t < half; t += 32) {
-      const int blk = t / hk, o = t - blk * hk;
+      const int blk = t >> lhk, o = t & ((1 << lhk) - 1);
       const int i = blk * k + o, p = blk * k + (k - 1 - o);
       if (p < n) { const int x = a[i], y = a[p]; if (x > y) { a[i] = y; a[p] = x; } }
     }
     __syncwarp();
-    for (int j = k >> 2; j > 0; j >>= 1) {
+    for (int lj = lk - 2; lj >= 0; --lj) {
+      const int j = 1 << lj;
       for (int t = lane; t < half; t += 32) {
-        const int i = (t / j) * 2 * j + (t % j), p = i + j;
+        const int i = ((t >> lj) << (lj + 1)) + (t & (j - 1)), p = i + j;
         if (p < n) { const int x = a[i], y = a[p]; if (x > y) { a[i] = y; a[p] = x; } }
       }
       __syncwarp();
@@ -462,8 +471,36 @@ __device__ __forceinline__ void solve_barrier(unsigned int* bar, unsigned int& e
   }
   __syncthreads();
 }
-__device__ __forceinline__ void dbg_max(const FastFrame& f, int k, long long v) { if (f.profile) atomicMax((unsigned long long*)&f.fc->dbg[k], (unsigned long long)v); }
-__device__ __forceinline__ void dbg_add(const FastFrame& f, int k, long long v) { if (f.profile) atomicAdd((unsigned long long*)&f.fc->dbg[k], (unsigned long long)v); }
+// Profiling probes of the solve kernel gather per CTA in shared memory and reach global memory once per CTA and phase (prof_flush):
+// one same-address global atomic per ray made the profiled frame 1.6x the timed one and moved the phases it measured.
+// Slots 0..15: FastCounters::dbg (kDbgAddMask: sums, the others maxima); 16, 17: maxima of prof[1], prof[2]; 18, 19: this sweep's
+// prof[4 + 2 i], prof[5 + 2 i].
+static constexpr int kDbgShared = 20;
+static constexpr unsigned kDbgAddMask = (1u << 4) | (1u << 5) | (1u << 6) | (1u << 7) | (1u << 9);
+__shared__ unsigned long long s_dbg[kDbgShared];
+__device__ __forceinline__ void dbg_max(const FastFrame& f, int k, long long v) { if (f.profile) atomicMax(&s_dbg[k], (unsigned long long)v); }
+__device__ __forceinline__ void dbg_add(const FastFrame& f, int k, long long v) { if (f.profile) atomicAdd(&s_dbg[k], (unsigned long long)v); }
+__device__ __forceinline__ void prof_init(const FastFrame& f) {
+  if (!f.profile) return;
+  if (threadIdx.x < kDbgShared) s_dbg[threadIdx.x] = 0;
+  __syncthreads();
+}
+// every thread of the CTA calls it before a grid barrier; `sweep_idx` is the index of the sweep that just ended (-1: none)
+__device__ __forceinline__ void prof_flush(const FastFrame& f, int sweep_idx) {
+  if (!f.profile) return;
+  __syncthreads();
+  const int k = threadIdx.x;
+  if (k < kDbgShared) {
+    const unsigned long long v = s_dbg[k];
+    if (v) {
+      if (k < 16) {
+        if ((kDbgAddMask >> k) & 1u) atomicAdd((unsigned long long*)&f.fc->dbg[k], v); else atomicMax((unsigned long long*)&f.fc->dbg[k], v);
+      } else if (k < 18) atomicMax((unsigned long long*)&f.prof[k - 15], v);
+      else if (sweep_idx >= 0 && sweep_idx < kProfSweeps) atomicAdd((unsigned long long*)&f.prof[4 + 2 * sweep_idx + (k - 18)], v);
+      s_dbg[k] = 0;
+    }
+  }
+}
 __device__ __forceinline__ void timeline_mark(const FastFrame& f, int slot) {
   if (f.profile && blockIdx.x == 0 && threadIdx.x == 0 && slot < kTimelineSlots) f.fc->timeline[slot] = clock64();
 }

@@ -67,22 +67,20 @@ __device__ __forceinline__ bool stamp_dirty(const Obs3& o, uint32_t slot, int la
 // first time a candidate turns performed: it enters the slot's bucket (or the overflow pool); returns its position code.
 // The overflow push is one exchange, no retry loop and no fence: a reader that catches the entry half-written (pending link, fields of
 // an older frame) takes a wrong decision for this sweep only - the inserter stamps the slot afterwards, which marks that reader dirty.
-__device__ __forceinline__ int cand_insert_raw(int* slot_cnt, uint64_t* bkt, int* head, OvfEnt* ovf, int ovf_cap, int* ovf_count, Counters* cnt,
-                                            uint32_t slot, uint64_t entry) {
-  const int idx = atomicAdd(&slot_cnt[slot], 1);
-  if (idx < kBkt3) { const int pos = (int)slot * kBkt3 + idx; __stcg(&bkt[pos], entry); return pos; }
-  const int id = atomicAdd(ovf_count, 1);
-  if (id >= ovf_cap) { set_err(cnt, 4); return -2; }
-  OvfEnt* e = &ovf[id];
+__device__ __forceinline__ int cand_insert3(const FastFrame& f, uint32_t slot, uint64_t entry) {
+  const Obs3& o = f.o3;
+  const int idx = atomicAdd(&o.slot_cnt[slot], 1);
+  if (f.profile) dbg_max(f, 16, idx + 1);
+  if (idx < kBkt3) { const int pos = (int)slot * kBkt3 + idx; __stcg(&o.bkt[pos], entry); return pos; }
+  const int id = atomicAdd(&f.fc->ovf_count, 1);
+  if (id >= o.ovf_cap) { set_err(f.cnt, 4); return -2; }
+  OvfEnt* e = &o.ovf[id];
   __stcg(&e->next, kOvfPending);
   __stcg(&e->order_perf, (entry & kEntPerf) | ((entry >> 13) & ((1ull << kEntOrderBits) - 1)));
   __stcg(&e->hi, (uint32_t)(entry & 0x1FFFull));
-  const int old = atomicExch(&head[slot], id);
+  const int old = atomicExch(&o.head[slot], id);
   __stcg(&e->next, old);
   return -3 - id;
-}
-__device__ __forceinline__ int cand_insert3(const FastFrame& f, uint32_t slot, uint64_t entry) {
-  return cand_insert_raw(f.o3.slot_cnt, f.o3.bkt, f.o3.head, f.o3.ovf, f.o3.ovf_cap, &f.fc->ovf_count, f.cnt, slot, entry);
 }
 
 // latest performed visit of `slot` that precedes `my_order`: its (value >> 20), or -1.  (A non-inlined variant of these helpers was measured
@@ -122,14 +120,28 @@ __device__ __forceinline__ int latest_performed_before3(const Obs3& o, uint32_t 
 }
 __device__ __forceinline__ bool later_performed_exists_raw(const uint64_t* bkt, const int* slot_cnt, const int* head, const OvfEnt* ovf, int ovf_cap,
                                                         uint32_t slot, uint64_t my_order) {
+  // the bucket is read 8 entries (4 x 16 B) per round trip, the first 8 independently of the count, as in latest_performed_before_raw:
+  // one dependent load per entry made the table commit as long as its slowest hot slot (up to 32 trips)
+  const ulonglong2* b = (const ulonglong2*)(bkt + (size_t)slot * kBkt3);
   const int total = __ldcg(&slot_cnt[slot]);
+  ulonglong2 v[4];
+#pragma unroll
+  for (int q = 0; q < 4; ++q) v[q] = __ldcg(b + q);
   const int n = total < kBkt3 ? total : kBkt3;
-  const uint64_t* b = bkt + (size_t)slot * kBkt3;
   bool later = false;
 #pragma unroll 1
-  for (int j = 0; j < n; ++j) {
-    const uint64_t e = __ldcg(&b[j]);
-    if ((e & kEntPerf) && ((e >> 13) & ((1ull << kEntOrderBits) - 1)) > my_order) later = true;
+  for (int q0 = 0;;) {
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const uint64_t e2[2] = {v[q].x, v[q].y};
+#pragma unroll
+      for (int k = 0; k < 2; ++k)
+        if (2 * (q0 + q) + k < n && (e2[k] & kEntPerf) && ((e2[k] >> 13) & ((1ull << kEntOrderBits) - 1)) > my_order) later = true;
+    }
+    q0 += 4;
+    if (2 * q0 >= n) break;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) v[q] = __ldcg(b + q0 + q);
   }
   if (total > kBkt3) {
     int guard = total - kBkt3 + 8;
@@ -299,7 +311,7 @@ __device__ __forceinline__ void fast3_sweep(const FastFrame& f, int sweep, int r
       }
       for (int d = 16; d > 0; d >>= 1) { const int t = __shfl_xor_sync(0xffffffffu, fd, d); fd = t < fd ? t : fd; }
     }
-    if (fd == 0x7fffffff) continue;
+    if (fd == 0x7fffffff) { if (f.profile && lane == 0) dbg_add(f, 18, 1); continue; }
     const long long t_eval = f.profile ? clock64() : 0;
     int n_blocks_eval = 0, n_blocks_mat = 0;
     int s0, blen;
@@ -370,6 +382,7 @@ __device__ __forceinline__ void fast3_sweep(const FastFrame& f, int sweep, int r
           const uint32_t stale = o.table[slot];   // issued together with the bucket loads
           const int hi = latest_performed_before3(o, slot, ((uint64_t)r << kOrderStepBits) | (uint64_t)s);
           coll[q] = (hi >= 0) ? ((uint32_t)hi == (uint32_t)(v[q] >> kSetBits)) : (stale == (uint32_t)(v[q] >> kSetBits));
+          if (f.profile) { const int tot = __ldcg(&o.slot_cnt[slot]); if (tot > kBkt3) dbg_max(f, 17, tot - kBkt3); }
         }
       }
       const unsigned bits0 = __ballot_sync(0xffffffffu, coll[0]), bits1 = __ballot_sync(0xffffffffu, coll[1]);
@@ -404,7 +417,7 @@ __device__ __forceinline__ void fast3_sweep(const FastFrame& f, int sweep, int r
     if (lane == 0) {
       if (U != old) { f.rayrec[r].L = U; cnt->changed[sweep & 3] = 1; }
       f.rayrec[r].eval_sweep = sweep;
-      if (f.profile) { dbg_max(f, 3, clock64() - t_eval); dbg_add(f, 4, 1); dbg_add(f, 5, n_blocks_eval); dbg_add(f, 6, n_blocks_mat); if (U != old) dbg_add(f, 7, 1); }
+      if (f.profile) { dbg_max(f, 3, clock64() - t_eval); dbg_add(f, 4, 1); dbg_add(f, 5, n_blocks_eval); dbg_add(f, 6, n_blocks_mat); if (U != old) dbg_add(f, 7, 1); dbg_add(f, 19, 1); }
     }
   }
 }
@@ -458,6 +471,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
   Counters* cnt = f.cnt;
   const int n_points = cnt->n_points;
   int tl = 0;
+  prof_init(f);
   timeline_mark(f, tl++);
   extern __shared__ int s_sort[];            // kSortPerWarp ints per warp
   // ---- phase 0a: start-set slots shared by several cells: every visitor files itself in the slot's list
@@ -469,6 +483,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
       const uint32_t slot = (uint32_t)v & kSetMask;
       if (f.s_hmin[slot] != f.s_hmax[slot]) f.m_list[f.s_base[slot] + f.sb.next[seq]] = seq;
     }
+    prof_flush(f, -1);
     solve_barrier(bar, epoch);
     timeline_mark(f, 57);
     // ---- phase 0b: one warp per such slot: visitors in sequence order; a visitor is cast iff its predecessor carried another value
@@ -479,16 +494,30 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
       const int n = __ldcg(&f.s_visits[slot]);
       int* seg = f.m_list + __ldcg(&f.s_base[slot]);
       int* a = seg;
-      if (n <= kSortPerWarp) { for (int i = lane; i < n; i += 32) scratch[i] = __ldcg(&seg[i]); a = scratch; }
+      if (n <= kSortPerWarp) {
+#pragma unroll 4
+        for (int i = lane; i < n; i += 32) scratch[i] = __ldcg(&seg[i]);
+        a = scratch;
+      }
       __syncwarp();
       warp_sort_i32(a, n, lane);
-      for (int i = 1 + lane; i < n; i += 32) {
-        const int pa = a[i - 1], pb = a[i];
-        if (f.pt_key[pa] != f.pt_key[pb]) { f.cast_flag[pb] = 1; atomicAdd(&f.warp_cnt[pb >> 5], 1); }
+      for (int i0 = 1 + lane; i0 < n; i0 += 4 * 32) {   // the keys of four neighbour pairs per lane in flight together
+        int pb[4];
+        uint64_t ka[4], kb[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const int i = i0 + 32 * u;
+          pb[u] = -1; ka[u] = kb[u] = 0;
+          if (i < n) { pb[u] = a[i]; ka[u] = f.pt_key[a[i - 1]]; kb[u] = f.pt_key[pb[u]]; }
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+          if (pb[u] >= 0 && ka[u] != kb[u]) { f.cast_flag[pb[u]] = 1; atomicAdd(&f.warp_cnt[pb[u] >> 5], 1); }
       }
       __syncwarp();
       if (f.profile && lane == 0) { dbg_max(f, 8, n); dbg_add(f, 9, n); }
     }
+    prof_flush(f, -1);
     solve_barrier(bar, epoch);
     timeline_mark(f, 58);
   }
@@ -498,6 +527,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
     const int total = block_scan_array(f.warp_cnt, f.warp_off, n_warps32);
     if (threadIdx.x == 0) cnt->n_cast = total;
   }
+  prof_flush(f, -1);
   solve_barrier(bar, epoch);
   timeline_mark(f, 59);
   const int n_cast = ((volatile int*)&cnt->n_cast)[0];
@@ -509,10 +539,12 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
   }
   const int sweep_base0 = ((volatile int*)&f.fc->sweep_base)[0];   // sweep ids are monotonic across frames (31 bits: never wraps in practice)
   const bool wrap = false;
+  prof_flush(f, -1);
   solve_barrier(bar, epoch);
   timeline_mark(f, tl++);
   // ---- phase 1: ray set-up (first kH0 steps of every ray)
   for (int r0 = (gtid & ~31); r0 < n_cast; r0 += gthreads) fast3_ray_setup(f, r0 + lane, n_cast);
+  prof_flush(f, -1);
   solve_barrier(bar, epoch);
   timeline_mark(f, tl++);
   // ---- phase 2: observed-set fixpoint, rank group by rank group
@@ -527,6 +559,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
     for (int it = 0; it < max_sweeps; ++it) {
       ++sweep;
       fast3_sweep(f, sweep, g_lo, g_hi, (WarpDdaScratch*)(s_sort + (threadIdx.x >> 5) * kSortPerWarp));
+      prof_flush(f, sweep - first_sweep);
       solve_barrier(bar, epoch);
       if (tl < kTimelineSlots - 12) timeline_mark(f, tl++);
       const int changed = ((volatile int*)cnt->changed)[sweep & 3];
@@ -549,6 +582,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
   timeline_mark(f, tl++);
   // ---- phase 3: table commit + block allocation + records per tile
   if (!failed) fast3_walk_performed<1>(f, n_cast, 0);
+  prof_flush(f, -1);
   solve_barrier(bar, epoch);
   timeline_mark(f, tl++);
   timeline_mark(f, tl++);     // (slot kept for the layout of k_fast_solve: there the per-tile count is a phase of its own)
@@ -576,6 +610,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
     }
   }
   if (ok) fast_block_init(f, n_new, pool_base);
+  prof_flush(f, -1);
   solve_barrier(bar, epoch);
   timeline_mark(f, tl++);
   // ---- phase 5: keys into the tile segments (the per-tile counters run back to zero: nothing to clear for the next frame)
@@ -590,6 +625,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) k_fast_solve3(FastFrame f, i
     f.fc->tile_cursor = 0;
     f.fc->n_tile_list = 0;
     f.fc->rec_cursor = 0;
+    if (f.profile) f.prof[0] = f.fc->ovf_count;
     f.fc->ovf_count = 0;
     if (f.profile) { f.fc->dbg[10] = n_mixed; f.fc->dbg[11] = n_cast; }
     f.fc->n_mixed = 0;
